@@ -19,6 +19,11 @@ overflow), no data-path collective, weak scaling; value = tokens/s summed over r
              qlinear_cuda_old.py:291-355) timed on this box's host cores on one decoder block.
 
 --impl reference times that CPU path alone (rank 0 only) and prints the same JSON shape.
+
+--dump-outputs DIR writes what the timed path returned in its last timed step as DIR/<name>.npy (float32, rank 0): y (the
+device-resident step) and y_e2e (the end-to-end step) of the decode workloads, y of the TP workload, one array per layer
+of the block the CPU arm times.  All inputs are seeded, so two builds run with the same arguments can be compared
+output for output.
 """
 from __future__ import annotations
 
@@ -69,6 +74,23 @@ def load_peaks():
         return json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json"))), "measured"
     except Exception:
         return {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0}, "fallback"
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(outdir, arrays):
+    """Save each tensor as float32 outdir/<name>.npy.  One that is larger than its share of DUMP_LIMIT_BYTES keeps a
+    fixed, seeded sample of its rows (the same rows on every run of the same workload)."""
+    os.makedirs(outdir, exist_ok=True)
+    share = DUMP_LIMIT_BYTES // max(1, len(arrays))
+    for name, t in arrays.items():
+        a = t.detach().float().cpu().numpy()
+        a = a.reshape(-1, a.shape[-1])
+        max_rows = max(1, (share - 4096) // (4 * a.shape[1]))
+        if a.shape[0] > max_rows:
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], max_rows, replace=False))]
+        np.save(os.path.join(outdir, f"{name}.npy"), a)
 
 
 # ------------------------------------------------------------------------------------------- clocks
@@ -240,8 +262,9 @@ def usable_cpus():
     return max(1, n)
 
 
-def cpu_block_time(hidden, inter, M, reps, threads):
-    """Reference CPU path on one decoder block (7 QuantLinear forwards).  Returns (seconds per block, sample text)."""
+def cpu_block_time(hidden, inter, M, reps, threads, outputs=None):
+    """Reference CPU path on one decoder block (7 QuantLinear forwards).  Returns (seconds per block, sample text);
+    `outputs`, when given, receives the layers' outputs of the last rep by layer name."""
     from oracle.ref_port_torch import python_fallback_forward
 
     torch.set_num_threads(threads)
@@ -255,8 +278,10 @@ def cpu_block_time(hidden, inter, M, reps, threads):
     xs = {K: torch.randn(M, K, generator=g) for K in (hidden, inter)}
 
     def run_block():
-        for (qw, qz, sc, K) in layers:
-            python_fallback_forward(xs[K], qw, qz, sc, GROUP)
+        for (name, _, _), (qw, qz, sc, K) in zip(block_shapes(hidden, inter), layers):
+            y = python_fallback_forward(xs[K], qw, qz, sc, GROUP)
+            if outputs is not None:
+                outputs[name] = y
 
     run_block()
     t0 = time.perf_counter()
@@ -296,10 +321,10 @@ def cpu_block_time_c(hidden, inter, M, reps):
         return None
 
 
-def cpu_block_time_qigen(hidden, inter, M, reps):
+def cpu_block_time_qigen(hidden, inter, M, reps, outputs=None):
     """The reference's own compiled CPU kernel (qigen, qlinear_qigen.py:257-338) on one decoder block, through
     oracle/qigen_ref.py around oracle/_ref/cQIGen (built from /root/reference by oracle/build_qigen.py; OpenMP thread count
-    baked in at generation time).  None when the library is not there."""
+    baked in at generation time).  None when the library is not there.  `outputs` as in cpu_block_time."""
     try:
         from oracle import qigen_ref
         if not qigen_ref.available():
@@ -318,8 +343,10 @@ def cpu_block_time_qigen(hidden, inter, M, reps):
         xs = {K: torch.from_numpy(rng.standard_normal((M, K)).astype(np.float32)) for K in (hidden, inter)}
 
         def run_block():
-            for lin in layers:
-                lin.forward(xs[lin.K])
+            for (name, _, _), lin in zip(block_shapes(hidden, inter), layers):
+                y = lin.forward(xs[lin.K])
+                if outputs is not None:
+                    outputs[name] = y
 
         run_block()
         t0 = time.perf_counter()
@@ -353,6 +380,7 @@ def run_reference(args, rank, world):
     threads = usable_cpus()
     Mc = cpu_rows_for(M)
     kind = "port"
+    outputs = {}
     probe = cpu_block_time_qigen(hidden, inter, Mc, 1)
     if probe is not None:
         # the reference's own compiled CPU kernel (qigen) - the strongest CPU implementation the reference has for this path
@@ -361,8 +389,8 @@ def run_reference(args, rank, world):
         times = []
         for _ in range(max(1, args.warmup)):
             cpu_block_time_qigen(hidden, inter, Mc, 1)
-        for _ in range(args.steps):
-            times.append(cpu_block_time_qigen(hidden, inter, Mc, 3)[0])
+        for i in range(args.steps):
+            times.append(cpu_block_time_qigen(hidden, inter, Mc, 3, outputs if i == args.steps - 1 else None)[0])
         sample = (f"1 of {n_blocks} decoder blocks (7 QuantLinear forwards, M={Mc}), the reference's qigen kernel "
                   f"(oracle/_ref/cQIGen, forward_gs4, {threads} OpenMP threads baked in), 3 reps per step")
     else:
@@ -370,8 +398,8 @@ def run_reference(args, rank, world):
             cpu_block_time(hidden, inter, Mc, 1, threads)
         times = []
         sample = ""
-        for _ in range(args.steps):
-            dt, sample = cpu_block_time(hidden, inter, Mc, 1, threads)
+        for i in range(args.steps):
+            dt, sample = cpu_block_time(hidden, inter, Mc, 1, threads, outputs if i == args.steps - 1 else None)
             times.append(dt)
     t_step = float(np.mean(times))                       # one block
     tokens_per_step = (Mc / n_blocks)                    # a block is 1/32 of a token's linears
@@ -386,6 +414,8 @@ def run_reference(args, rank, world):
         "e2e": {"value": value, "unit": "tokens/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     print(json.dumps(line), flush=True)
 
 
@@ -395,6 +425,7 @@ def run_b200(args, rank, world, local_rank):
     hidden, inter, n_blocks, M, desc = WORKLOADS[args.workload]
     dev = torch.device("cuda", local_rank)
     torch.cuda.set_device(dev)
+    torch.manual_seed(4321 + rank)                       # activations: the same inputs on every run
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
     from autogptq_b200 import _lib
@@ -497,6 +528,7 @@ def run_b200(args, rank, world, local_rank):
         ms_dev = timed(g_dev, args.steps)
         t1 = time.time()
         clocks = sampler.stop(t0, t1) if rank == 0 else None
+        outputs = {"y": (ch_y if use_chain else y_dev).clone()}      # the e2e graph below overwrites ch_y
 
         feed = [torch.randn(M, hidden, dtype=torch.float16) for _ in range(4)]
         checksum = [0.0]
@@ -509,6 +541,7 @@ def run_b200(args, rank, world, local_rank):
         for i in range(max(3, args.warmup)):
             host_step(i); g_e2e.replay(); stream.synchronize()
         ms_e2e = timed(g_e2e, args.steps, host_step)
+        outputs["y_e2e"] = y_host.clone()
 
     tokens_per_step = M * world                          # weak scaling: every rank decodes its own stream
     value = tokens_per_step / (ms_dev / args.steps / 1e3)
@@ -619,6 +652,8 @@ def run_b200(args, rank, world, local_rank):
         if c_arm is not None:       # extra information: a compiled CPU arm next to the reference's python path
             line["cpu_baseline_c"] = {"value": (cpu_rows_for(M) / n_blocks) / c_arm[0], "unit": "tokens/s", "cores": c_arm[1],
                                       "kind": "port", "sample": "same block, C / OpenMP restatement (qigen-style sum(x) formulation), 3 reps"}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -659,10 +694,11 @@ def build_tp_blocks(hidden, inter, kv, n_blocks, rank, world, dev, log=None):
     return blocks
 
 
-def tp_chain_record(args, rank, world, local_rank, n_blocks=None, steps=None):
+def tp_chain_record(args, rank, world, local_rank, n_blocks=None, steps=None, outputs=None):
     """Llama-2-70B decode, QuantLinears column/row-sharded over `world` ranks (BASELINE configs[3]): one persistent
     chain launch per rank and token, the row-parallel all-reduces fused into it (tagged words over NVLink peer memory,
-    autogptq_b200.tp.TPDecodeChain), replayed as a CUDA graph.  Returns the record (rank 0) or None."""
+    autogptq_b200.tp.TPDecodeChain), replayed as a CUDA graph.  Returns the record (rank 0) or None; `outputs`, when
+    given, receives the output of the last timed step as "y"."""
     import torch.distributed as dist
     from autogptq_b200.tp import TPDecodeChain
 
@@ -703,6 +739,8 @@ def tp_chain_record(args, rank, world, local_rank, n_blocks=None, steps=None):
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev, dtype=torch.float64)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
+        if outputs is not None:
+            outputs["y"] = tp.output().clone()
     ms = float(ms.item())
     info = tp.chain.info()
     del tp, blocks
@@ -729,13 +767,15 @@ def run_tp(args, rank, world, local_rank):
 
     dev = torch.device("cuda", local_rank)
     torch.cuda.set_device(dev)
+    torch.manual_seed(4321)                              # the TP input: the same on every rank and run
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
     t0 = time.time()
-    rec = tp_chain_record(args, rank, world, local_rank, steps=args.steps)
+    outputs = {}
+    rec = tp_chain_record(args, rank, world, local_rank, steps=args.steps, outputs=outputs)
     t1 = time.time()
     if rank == 0:
         clocks = sampler.stop(t0, t1)
@@ -754,6 +794,8 @@ def run_tp(args, rank, world, local_rank):
                          "note": "per-rank algorithmic bytes / step time; the step contains the fused all-reduces"},
             "clocks": clocks,
         }
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -769,6 +811,8 @@ def main():
     ap.add_argument("--prefetch", action="store_true", help="switch the learned next-layer L2 prefetch of decode launches on (experiment; measured slower)")
     ap.add_argument("--siblings", default="chain", choices=["chain", "group", "branches", "serial"],
                     help="how the token's layers are issued: chain = the whole token as one persistent launch (decode, M <= 2); otherwise per-layer launches with sibling layers (q|k|v, gate|up) as one grouped launch, parallel graph branches, or serially")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the timed path returned in its last step as DIR/<name>.npy (float32)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -1,4 +1,6 @@
 """Shared helpers for the parity tests (the oracle is imported here and only here / in tests)."""
+import hashlib
+
 import numpy as np
 import torch
 
@@ -50,6 +52,14 @@ def assert_parity(y, y_ref, rtol=1e-3, atol_rms=1e-3, what=""):
                           f"rms(ref)={rms:.4e}, max|ref|={np.abs(y_ref).max():.4e}")
     # fp16 output rounding alone is 2^-11 * max|ref|; the band below is that plus the 1e-3 budget
     assert err.max() <= 1.5 * rtol * np.abs(y_ref).max() + 1e-6, f"{what}: max abs err {err.max():.4e}"
+
+
+def digest(*arrays) -> str:
+    """Fingerprint of the seeded inputs a stored (golden) output was computed from."""
+    h = hashlib.sha256()
+    for a in arrays:
+        h.update(np.ascontiguousarray(a).tobytes())
+    return h.hexdigest()
 
 
 def rand_x(M, K, seed=1, dtype=np.float16):

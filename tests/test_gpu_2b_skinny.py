@@ -1,10 +1,12 @@
 """GPU parity: the skinny (M <= 8) decode kernel through the QuantLinear module / C ABI vs the oracle."""
+import os
+
 import numpy as np
 import pytest
 import torch
 
 from oracle import w4a16_oracle as O
-from tests._util import assert_parity, make_layer, oracle_exact, rand_x
+from tests._util import assert_parity, digest, make_layer, oracle_exact, rand_x
 
 pytestmark = pytest.mark.gpu
 SKINNY = 3
@@ -79,21 +81,33 @@ def test_skinny_agrees_with_gemv_bitwise_tolerance():
     assert_parity(y_s, y_v, rtol=1e-3, atol_rms=6e-4, what="skinny vs gemv")
 
 
-def test_reference_exllamav2_kernel_agrees():
-    """The reference's own default 4-bit CUDA kernel (compiled from /root/reference into oracle/_ref by
-    oracle/build_ref.py) on the same packed buffers - tolerance of tests/test_q4.py:1120,1941."""
+EXLLAMAV2_CASE = dict(K=1024, N=1024, g=128, seed=43, Ms=(1, 8, 64))
+
+
+def exllamav2_inputs():
+    c = EXLLAMAV2_CASE
+    return O.random_packed(c["K"], c["N"], c["g"], seed=c["seed"]), {M: rand_x(M, c["K"], seed=M) for M in c["Ms"]}
+
+
+def test_reference_exllamav2_kernel_agrees(golden_dir):
+    """The reference's own default 4-bit CUDA kernel on the same packed buffers - tolerance of tests/test_q4.py:1120,1941.
+    Its outputs on these seeded inputs are stored in tests/golden/exllamav2_outputs.npz (tests/golden/make_golden_kernels.py);
+    where oracle/_ref/exllamav2_kernels has been built (oracle/build_ref.py), the live kernel is checked as well."""
     from oracle import ref_kernels
 
-    if ref_kernels.exllamav2() is None:
-        pytest.skip("oracle/_ref/exllamav2_kernels not built")
-    K, N, g = 1024, 1024, 128
-    d = O.random_packed(K, N, g, seed=43)
+    K, N = EXLLAMAV2_CASE["K"], EXLLAMAV2_CASE["N"]
+    d, xs = exllamav2_inputs()
+    stored = np.load(os.path.join(golden_dir, "exllamav2_outputs.npz"))
+    assert str(stored["digest"]) == digest(d["qweight"], d["qzeros"], d["scales"], *xs.values()), "seeded inputs changed"
     lin = make_layer(d)
-    ref = ref_kernels.ExllamaV2Layer(lin.qweight, lin.qzeros, lin.scales, K, N)
-    for M in (1, 8, 64):
-        x = torch.from_numpy(rand_x(M, K, seed=M)).cuda()
+    live = ref_kernels.ExllamaV2Layer(lin.qweight, lin.qzeros, lin.scales, K, N) if ref_kernels.exllamav2() else None
+    for M, xh in xs.items():
+        x = torch.from_numpy(xh).cuda()
         y = lin(x).float()
-        y_ref = ref(x).float()
+        refs = {"stored": torch.from_numpy(stored[f"y_{M}"]).cuda().float()}
+        if live is not None:
+            refs["live"] = live(x).float()
         torch.cuda.synchronize()
-        rms = y_ref.pow(2).mean().sqrt().item()
-        assert (y - y_ref).abs().max().item() <= 1e-2 * rms + 2e-2, f"M={M}"
+        for what, y_ref in refs.items():
+            rms = y_ref.pow(2).mean().sqrt().item()
+            assert (y - y_ref).abs().max().item() <= 1e-2 * rms + 2e-2, f"M={M} ({what})"

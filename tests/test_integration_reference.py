@@ -1,19 +1,17 @@
 """J1 - "AutoGPTQForCausalLM loads and runs unchanged": the B200 QuantLinear through the reference's OWN construction
 path.
 
-CPU part (runs where /root/reference is mounted): the reference's `modeling/_utils.py` is imported UNMODIFIED by file
-path - `accelerate` is absent in this image, so a stub stands in for it and the package `__init__`s (which pull in the
-whole model zoo) are bypassed with namespace stand-ins, exactly the technique SURVEY.md 8c used for gekko - then
-`patch_auto_gptq()` rebinds the selection point and the reference's `make_quant` (_utils.py:69-148: positional
-constructor, `new_layer.device = ...; .to(device)`), the name-keyed buffer fill (_base.py:1114-1121) and
-`autogptq_post_init` (_utils.py:380-513) run on a tiny HF Llama.
+CPU part: replays what the reference's `modeling/_utils.py` did when it built this package's module, as recorded from the
+unmodified original by tests/golden/make_golden_integration.py into tests/golden/ref_make_quant.json: the selection call
+that `patch_auto_gptq()` answers, `make_quant`'s positional constructor calls (_utils.py:69-148) with `new_layer.device =
+...; .to(device)`, then the name-keyed buffer fill (_base.py:1114-1121) on a tiny HF Llama; `autogptq_post_init`
+(_utils.py:380-513) must not act on our QUANT_TYPE.
 
-GPU part (no reference on the GPU box): the same construction sequence written out, a GPTQ checkpoint written with
+GPU part: the same construction sequence written out, a GPTQ checkpoint written with
 `QuantLinear.pack` to safetensors and read back (also through `autogptq_b200.checkpoint`), logits and greedy decode
 (reference tests/test_q4.py:1165-1222 compares generated text) against the same model holding the dequantised fp16
 weights in plain nn.Linear."""
-import importlib
-import importlib.util
+import json
 import os
 import sys
 import types
@@ -23,7 +21,7 @@ import pytest
 import torch
 import torch.nn as nn
 
-REF = "/root/reference/auto_gptq"
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 LINEAR_NAMES = ("q_proj", "k_proj", "v_proj", "o_proj", "gate_proj", "up_proj", "down_proj")
 
 
@@ -67,63 +65,60 @@ def _rtn_pack(model, group_size=128):
     return packed, deq
 
 
-def _import_reference_utils():
-    """auto_gptq.modeling._utils of the reference, unmodified, without running the package __init__s."""
-    if "accelerate" not in sys.modules:
-        import importlib.machinery
-
-        acc = types.ModuleType("accelerate")
-        acc.__path__ = []
-        acc.__spec__ = importlib.machinery.ModuleSpec("accelerate", None, is_package=True)
-        acc.__agb200_stub__ = True
-        acc_utils = types.ModuleType("accelerate.utils")
-        acc_utils.__spec__ = importlib.machinery.ModuleSpec("accelerate.utils", None)
-        acc.utils = acc_utils
-        sys.modules["accelerate"], sys.modules["accelerate.utils"] = acc, acc_utils
-    for pkg, sub in (("auto_gptq", ""), ("auto_gptq.modeling", "modeling"), ("auto_gptq.utils", "utils"),
-                     ("auto_gptq.nn_modules", "nn_modules"), ("auto_gptq.nn_modules.qlinear", "nn_modules/qlinear")):
-        if pkg not in sys.modules:
-            m = types.ModuleType(pkg)
-            m.__path__ = [os.path.join(REF, sub)] if sub else [REF]
-            sys.modules[pkg] = m
-    return importlib.import_module("auto_gptq.modeling._utils")
+def _stand_in_auto_gptq():
+    """An importable `auto_gptq.modeling._utils` that binds `dynamically_import_QuantLinear` by name, as the original
+    does at import time (_utils.py:17); returns it."""
+    for pkg in ("auto_gptq", "auto_gptq.modeling"):
+        sys.modules[pkg] = types.ModuleType(pkg)
+        sys.modules[pkg].__path__ = []
+    utils = types.ModuleType("auto_gptq.modeling._utils")
+    utils.dynamically_import_QuantLinear = None
+    sys.modules[utils.__name__] = utils
+    return utils
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not mounted")
 def test_reference_make_quant_builds_and_fills_the_b200_module():
     import autogptq_b200
     from autogptq_b200 import QuantLinear
 
-    model = _tiny_llama()                      # imports transformers before the accelerate stand-in exists
+    with open(os.path.join(GOLDEN, "ref_make_quant.json")) as f:
+        rec = json.load(f)
+    model = _tiny_llama()
     packed, _ = _rtn_pack(model)
-    U = _import_reference_utils()
-    patched = autogptq_b200.patch_auto_gptq()
-    assert "auto_gptq.modeling._utils" in patched
+    names = _quant_names(model)
+    assert [layer["name"] for layer in rec["layers"]] == names and len(names) == 14
     try:
-        names = _quant_names(model)
-        # the reference's own construction path (modeling/_utils.py:69-148), backend flags as from_quantized passes them
-        U.make_quant(model, names, 4, 128, use_triton=False, disable_exllama=True, disable_exllamav2=False,
-                     use_cuda_fp16=True, desc_act=False, trainable=False)
-        mods = dict(model.named_modules())
-        assert all(isinstance(mods[n], QuantLinear) for n in names) and len(names) == 14
-        assert all(hasattr(mods[n], "device") for n in names)           # `new_layer.device = ori_layer_device`
-        # name-keyed buffer fill (what accelerate.load_checkpoint_in_model does with the checkpoint keys, _base.py:1114-1121)
-        sd = {f"{n}.{k}": v for n, q in packed.items() for k, v in q.state_dict().items()}
-        missing, unexpected = model.load_state_dict(sd, strict=False)
-        assert not unexpected and not [m for m in missing if any(x in m for x in ("qweight", "qzeros", "scales", "g_idx"))]
-        for n in names:
-            assert torch.equal(mods[n].qweight, packed[n].qweight) and torch.equal(mods[n].scales, packed[n].scales)
-        # autogptq_post_init walks the modules by QUANT_TYPE (_utils.py:380-513): ours is none of its own, nothing breaks
-        assert U.autogptq_post_init(model, use_act_order=False) is model
-        # no CPU fallback in the product: a forward without a GPU fails loudly
-        with pytest.raises(RuntimeError):
-            mods[names[0]](torch.zeros(1, 256, dtype=torch.float16))
+        U = _stand_in_auto_gptq()
+        assert "auto_gptq.modeling._utils" in autogptq_b200.patch_auto_gptq()
+        # the selection make_quant made (backend flags as from_quantized passes them)
+        assert rec["selections"] and all(U.dynamically_import_QuantLinear(**sel) is QuantLinear for sel in rec["selections"])
     finally:
         for name in list(sys.modules):
             if name == "auto_gptq" or name.startswith("auto_gptq."):
                 del sys.modules[name]
-        if getattr(sys.modules.get("accelerate"), "__agb200_stub__", False):
-            del sys.modules["accelerate"], sys.modules["accelerate.utils"]
+    # make_quant's construction of every layer: positional ctor, `new_layer.device = ori_layer_device`, .to(), setattr
+    for layer in rec["layers"]:
+        kwargs = {k: getattr(torch, v.removeprefix("torch.")) if k == "weight_dtype" else v for k, v in layer["kwargs"].items()}
+        new = QuantLinear(*layer["args"], **kwargs)
+        new.device = torch.device(layer["device"])
+        for args in layer["to"]:
+            new = new.to(*(torch.device(a) for a in args))
+        parent_name, _, child = layer["name"].rpartition(".")
+        setattr(model.get_submodule(parent_name), child, new)
+    mods = dict(model.named_modules())
+    assert all(isinstance(mods[n], QuantLinear) for n in names)
+    assert all(hasattr(mods[n], "device") for n in names)
+    # name-keyed buffer fill (what accelerate.load_checkpoint_in_model does with the checkpoint keys, _base.py:1114-1121)
+    sd = {f"{n}.{k}": v for n, q in packed.items() for k, v in q.state_dict().items()}
+    missing, unexpected = model.load_state_dict(sd, strict=False)
+    assert not unexpected and not [m for m in missing if any(x in m for x in ("qweight", "qzeros", "scales", "g_idx"))]
+    for n in names:
+        assert torch.equal(mods[n].qweight, packed[n].qweight) and torch.equal(mods[n].scales, packed[n].scales)
+    # autogptq_post_init walks the modules by QUANT_TYPE (_utils.py:380-513): ours is none of those it handles
+    assert rec["post_init_acts_on"] and QuantLinear.QUANT_TYPE not in rec["post_init_acts_on"]
+    # no CPU fallback in the product: a forward without a GPU fails loudly
+    with pytest.raises(RuntimeError):
+        mods[names[0]](torch.zeros(1, 256, dtype=torch.float16))
 
 
 @pytest.mark.gpu
