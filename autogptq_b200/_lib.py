@@ -18,7 +18,7 @@ CHAIN_MAX_M = 2
 CHAIN_X_PLAIN, CHAIN_X_SILU_MUL, CHAIN_X_SUM_PARTS = 0, 1, 2
 CHAIN_DEBUG_NO_DEPS, CHAIN_DEBUG_NO_MATH = 1, 2
 PEER_HANDLE_BYTES = 64
-KERNEL_AUTO, KERNEL_GEMV, KERNEL_GEMM, KERNEL_SKINNY, KERNEL_DECODE, KERNEL_TCDECODE, KERNEL_IMMA = 0, 1, 2, 3, 4, 5, 6
+KERNEL_AUTO, KERNEL_GEMV, KERNEL_GEMM, KERNEL_SKINNY, KERNEL_IMMA = 0, 1, 2, 3, 6
 GEMV_MAX_M = 4
 SKINNY_MAX_M = 8
 IMMA_MAX_M = 8

@@ -26,8 +26,6 @@ NVCC_FLAGS = [
     "-Xcompiler", "-fPIC",
     "-DAGB200_NO_FAST_MATH",
 ]
-if os.environ.get("AGB200_EXPERIMENTAL", "0") == "1":      # the three decode kernel families AUTO never selects (DESIGN.md 3.6)
-    NVCC_FLAGS.append("-DAGB200_EXPERIMENTAL_KERNELS")
 # translation units of the library (compiled in parallel, then linked)
 UNITS = ["abi.cu", "chain.cu"]
 # chain.cu holds only the 576-thread persistent chain kernel: 65536 / 576 = 113 registers per thread at most

@@ -17,14 +17,6 @@
 #include "skinny.cuh"
 #include "decode_imma.cuh"
 #include "decode_imma_persistent.cuh"
-// Three decode kernel families that AUTO never selects (honest negative results of round 1: TMA-staged mma.sync decode,
-// tcgen05 small-N decode, TMA-staged IMMA decode - DESIGN.md 3.6) are only compiled with -DAGB200_EXPERIMENTAL_KERNELS
-// (`AGB200_EXPERIMENTAL=1 python -m autogptq_b200.build`); a default build answers AGB200_ENOSUP for them.
-#ifdef AGB200_EXPERIMENTAL_KERNELS
-#include "decode_tma.cuh"
-#include "decode_tc.cuh"
-#include "decode_imma_tma.cuh"
-#endif
 
 namespace {
 
@@ -55,6 +47,11 @@ int fail(int code, const char* fmt, ...) {
     cudaError_t e_ = (expr);                                                                   \
     if (e_ != cudaSuccess) return fail(AGB200_ECUDA, "%s: %s", #expr, cudaGetErrorString(e_)); \
   } while (0)
+
+// 0, or the AGB200_ECUDA failure of a kernel launch through agb::launch
+int launch_status(cudaError_t e, const char* what) {
+  return e == cudaSuccess ? 0 : fail(AGB200_ECUDA, "%s launch: %s", what, cudaGetErrorString(e));
+}
 
 bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
@@ -102,39 +99,15 @@ using agb::GemvParams;
 
 template <int kM, int kLN, bool kBf16, bool kBiased, int kOcc = 2>
 int launch_gemv_inst(const GemvParams& p, int n_tiles, cudaStream_t stream, int smem_optin) {
-  auto kern = agb::w4a16_gemv_kernel<kM, kLN, kBf16, kBiased, (kM == 1 ? kOcc : (kM <= 2 ? 2 : 1))>;
   const size_t smem = agb::GemvSmem<kM, kLN, kBiased>::total(p.rows_per_split);
   if (smem > static_cast<size_t>(smem_optin))
     return fail(AGB200_ENOSUP, "gemv: K chunk of %d rows needs %zu B shared memory (> %d)", p.rows_per_split, smem, smem_optin);
-  static bool attr_set_dev[64] = {};   // cudaFuncSetAttribute is per device; benign race: idempotent
-  const int attr_dev = agb::current_device_index();
-  if (!attr_set_dev[attr_dev]) {
-    AGB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_optin));
-    attr_set_dev[attr_dev] = true;
-  }
   GemvParams pp = p;
   agb::prefetch_set_grid(pp.pf, static_cast<unsigned>(n_tiles) * p.split);
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(n_tiles, p.split, 1);
-  cfg.blockDim = dim3(agb::kGemvThreads, 1, 1);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attrs[2];
-  int na = 0;
-  attrs[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attrs[na].val.programmaticStreamSerializationAllowed = pdl_allowed();
-  ++na;
-  if (p.split > 1) {
-    attrs[na].id = cudaLaunchAttributeClusterDimension;
-    attrs[na].val.clusterDim.x = 1;
-    attrs[na].val.clusterDim.y = p.split;
-    attrs[na].val.clusterDim.z = 1;
-    ++na;
-  }
-  cfg.attrs = attrs;
-  cfg.numAttrs = na;
-  AGB_CUDA(cudaLaunchKernelEx(&cfg, kern, pp));
-  return 0;
+  return launch_status(agb::launch<agb::w4a16_gemv_kernel<kM, kLN, kBf16, kBiased, (kM == 1 ? kOcc : (kM <= 2 ? 2 : 1))>>(
+                           dim3(n_tiles, p.split), dim3(agb::kGemvThreads), smem, smem_optin, pdl_allowed(), dim3(1, p.split),
+                           false, stream, pp),
+                       "gemv");
 }
 
 template <int kM, int kLN>
@@ -214,37 +187,13 @@ int gemv_pass(const void* x, const int32_t* qweight, const int32_t* qzeros, cons
 // ------------------------------------------------------------------------------------------ skinny (M <= 8)
 template <bool kBf16, bool kBiased>
 int launch_skinny_inst(const agb::SkinnyParams& p, cudaStream_t stream, int smem_optin) {
-  auto kern = agb::w4a16_skinny_kernel<kBf16, kBiased>;
   const size_t smem = agb::SkinnySmem::total(p.rows_per_split, p.M);
   if (smem > static_cast<size_t>(smem_optin))
     return fail(AGB200_ENOSUP, "skinny: K chunk of %d rows x M=%d needs %zu B shared memory (> %d)", p.rows_per_split, p.M, smem, smem_optin);
-  static bool attr_set_dev[64] = {};   // cudaFuncSetAttribute is per device; benign race: idempotent
-  const int attr_dev = agb::current_device_index();
-  if (!attr_set_dev[attr_dev]) {
-    AGB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_optin));
-    attr_set_dev[attr_dev] = true;
-  }
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((p.N + agb::kSkTN - 1) / agb::kSkTN, p.split, 1);
-  cfg.blockDim = dim3(agb::kSkThreads, 1, 1);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attrs[2];
-  int na = 0;
-  attrs[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attrs[na].val.programmaticStreamSerializationAllowed = pdl_allowed();
-  ++na;
-  if (p.split > 1) {
-    attrs[na].id = cudaLaunchAttributeClusterDimension;
-    attrs[na].val.clusterDim.x = 1;
-    attrs[na].val.clusterDim.y = p.split;
-    attrs[na].val.clusterDim.z = 1;
-    ++na;
-  }
-  cfg.attrs = attrs;
-  cfg.numAttrs = na;
-  AGB_CUDA(cudaLaunchKernelEx(&cfg, kern, p));
-  return 0;
+  return launch_status(agb::launch<agb::w4a16_skinny_kernel<kBf16, kBiased>>(
+                           dim3((p.N + agb::kSkTN - 1) / agb::kSkTN, p.split), dim3(agb::kSkThreads), smem, smem_optin,
+                           pdl_allowed(), dim3(1, p.split), false, stream, p),
+                       "skinny");
 }
 
 int skinny_launch(const void* x, const int32_t* qweight, const int32_t* qzeros, const void* scales, const int32_t* perm,
@@ -271,122 +220,31 @@ int skinny_launch(const void* x, const int32_t* qweight, const int32_t* qzeros, 
   return launch_skinny_inst<false, false>(p, stream, di.smem_optin);
 }
 
-#ifdef AGB200_EXPERIMENTAL_KERNELS
-// ------------------------------------------------------------------------------------------ decode (TMA-staged, M <= 8)
-template <bool kBf16>
-int launch_decode_inst(const agb::DecodeParams& p, const CUtensorMap& tmap, int grid, size_t smem, cudaStream_t stream, int smem_optin) {
-  auto kern = agb::w4a16_decode_kernel<kBf16>;
-  static bool attr_set_dev[64] = {};   // cudaFuncSetAttribute is per device; benign race: idempotent
-  const int attr_dev = agb::current_device_index();
-  if (!attr_set_dev[attr_dev]) {
-    AGB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_optin));
-    attr_set_dev[attr_dev] = true;
+// Fills the layer table of a grouped launch: sibling layers that read the same x each own ceil(N[i] / tile_n)
+// consecutive tiles of the grid.  Returns the number of tiles.
+int fill_layers(agb::GemvLayerRef* layer, int n_layers, const int32_t* const* qweight, const int32_t* const* qzeros,
+                const void* const* scales, const int32_t* const* perm, const void* const* bias, void* const* y,
+                const int* N, int tile_n) {
+  int tiles = 0;
+  for (int i = 0; i < n_layers; ++i) {
+    layer[i].qweight = qweight[i]; layer[i].qzeros = qzeros[i]; layer[i].scales = scales[i];
+    layer[i].perm = perm ? perm[i] : nullptr; layer[i].bias = bias ? bias[i] : nullptr; layer[i].y = y[i];
+    layer[i].N = N[i]; layer[i].tile_begin = tiles;
+    tiles += (N[i] + tile_n - 1) / tile_n;
   }
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(grid, 1, 1);
-  cfg.blockDim = dim3(agb::kDcThreads, 1, 1);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attrs[1];
-  attrs[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attrs[0].val.programmaticStreamSerializationAllowed = pdl_allowed();
-  cfg.attrs = attrs;
-  cfg.numAttrs = 1;
-  AGB_CUDA(cudaLaunchKernelEx(&cfg, kern, p, tmap));
-  return 0;
+  return tiles;
 }
-
-int decode_launch(const void* x, const int32_t* qweight, const int32_t* qzeros, const void* scales, const int32_t* perm,
-                  const void* bias, void* y, int M, int K, int N, int group_size, bool bf16, int grid_req, int stages_req,
-                  cudaStream_t stream, const DeviceInfo& di) {
-  if (group_size % 32 != 0) return fail(AGB200_ENOSUP, "decode kernel needs group_size %% 32 == 0 (got %d)", group_size);
-  if (M < 1 || M > agb::kDcMaxM) return fail(AGB200_EINVAL, "decode kernel handles 1 <= M <= 8 (got %d)", M);
-  agb::DecodeParams p{};
-  p.x = x; p.qzeros = qzeros; p.scales = scales; p.perm = perm; p.bias = bias; p.y = y;
-  p.M = M; p.K = K; p.N = N; p.rows = K / 8; p.rows_per_group = group_size / 8;
-  p.num_tiles = (N + agb::kDcTN - 1) / agb::kDcTN;
-  p.num_chunks = (p.rows + agb::kDcStageRows - 1) / agb::kDcStageRows;
-  p.rows_pad = p.num_chunks * agb::kDcStageRows;
-  p.rpg_log2 = -1;
-  for (int b = 2; b < 24; ++b) if (p.rows_per_group == (1 << b)) p.rpg_log2 = b;
-  if (group_size >= K) p.rpg_log2 = 30;                       // single group
-  if (p.rpg_log2 < 0) return fail(AGB200_ENOSUP, "decode kernel needs a power-of-two group_size (got %d)", group_size);
-  // balanced persistent grid: every CTA owns the same number of column tiles (+-1)
-  int grid = grid_req;
-  if (grid <= 0) {
-    const int waves = (p.num_tiles + di.sms - 1) / di.sms;
-    grid = (p.num_tiles + waves - 1) / waves;
-  }
-  if (grid > p.num_tiles) grid = p.num_tiles;
-  const int tiles_per_cta = (p.num_tiles + grid - 1) / grid;
-  // ring depth: never more than the CTA will consume; keep the CTA under half an SM when x is small so that
-  // two consecutive layers are co-resident (PDL), otherwise take what is left
-  const size_t fixed = agb::DecodeSmem::total(0, p.rows, M);
-  const size_t half_sm = 110 * 1024;
-  int stages = stages_req;
-  if (stages <= 0) {
-    const size_t budget = fixed + 2 * agb::kDcStageBytes <= half_sm ? half_sm : static_cast<size_t>(di.smem_optin);
-    stages = static_cast<int>((budget - fixed) / agb::kDcStageBytes);
-  }
-  if (stages > agb::kDcMaxStages) stages = agb::kDcMaxStages;
-  if (stages > p.num_chunks * tiles_per_cta) stages = p.num_chunks * tiles_per_cta;
-  if (stages < 1) stages = 1;
-  p.stages = stages;
-  const size_t smem = agb::DecodeSmem::total(stages, p.rows, M);
-  if (smem > static_cast<size_t>(di.smem_optin))
-    return fail(AGB200_ENOSUP, "decode: K=%d x M=%d needs %zu B shared memory (> %d)", K, M, smem, di.smem_optin);
-
-  agb::EncodeTiledFn encode = agb::get_encode_fn();
-  if (encode == nullptr) return fail(AGB200_ECUDA, "cuTensorMapEncodeTiled entry point not available");
-  CUtensorMap tmap;
-  const cuuint64_t gdim[2] = {static_cast<cuuint64_t>(N), static_cast<cuuint64_t>(p.rows)};
-  const cuuint64_t gstride[1] = {static_cast<cuuint64_t>(N) * 4};
-  const cuuint32_t box[2] = {static_cast<cuuint32_t>(agb::kDcTN), static_cast<cuuint32_t>(agb::kDcStageRows)};
-  const cuuint32_t estr[2] = {1, 1};
-  CUresult cr = encode(&tmap, CU_TENSOR_MAP_DATA_TYPE_INT32, 2, const_cast<int32_t*>(qweight), gdim, gstride, box, estr,
-                       CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                       CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (cr != CUDA_SUCCESS) return fail(AGB200_ECUDA, "cuTensorMapEncodeTiled(qweight) failed (CUresult %d)", static_cast<int>(cr));
-  return bf16 ? launch_decode_inst<true>(p, tmap, grid, smem, stream, di.smem_optin)
-              : launch_decode_inst<false>(p, tmap, grid, smem, stream, di.smem_optin);
-}
-
-#endif  // AGB200_EXPERIMENTAL_KERNELS
 
 // ------------------------------------------------------------------------------------------ integer tensor-core decode (M <= 8)
 template <int kNG, int kWN, bool kBf16>
 int launch_imma_inst(const agb::ImmaParams& p, int n_tiles, cudaStream_t stream, int smem_optin) {
-  auto kern = agb::w4a16_imma_kernel<kNG, kWN, kBf16>;
   const size_t smem = agb::ImmaSmem::total(p.rows_per_split, p.M, 8 * kNG, 32 * kWN);
   if (smem > static_cast<size_t>(smem_optin))
     return fail(AGB200_ENOSUP, "imma: K chunk of %d rows x M=%d needs %zu B shared memory (> %d)", p.rows_per_split, p.M, smem, smem_optin);
-  static bool attr_set_dev[64] = {};   // cudaFuncSetAttribute is per device; benign race: idempotent
-  const int attr_dev = agb::current_device_index();
-  if (!attr_set_dev[attr_dev]) {
-    AGB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_optin));
-    attr_set_dev[attr_dev] = true;
-  }
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(n_tiles, p.split, 1);
-  cfg.blockDim = dim3(agb::kImThreads, 1, 1);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attrs[2];
-  int na = 0;
-  attrs[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attrs[na].val.programmaticStreamSerializationAllowed = pdl_allowed();
-  ++na;
-  if (p.split > 1) {
-    attrs[na].id = cudaLaunchAttributeClusterDimension;
-    attrs[na].val.clusterDim.x = 1;
-    attrs[na].val.clusterDim.y = p.split;
-    attrs[na].val.clusterDim.z = 1;
-    ++na;
-  }
-  cfg.attrs = attrs;
-  cfg.numAttrs = na;
-  AGB_CUDA(cudaLaunchKernelEx(&cfg, kern, p));
-  return 0;
+  return launch_status(agb::launch<agb::w4a16_imma_kernel<kNG, kWN, kBf16>>(dim3(n_tiles, p.split), dim3(agb::kImThreads), smem,
+                                                                           smem_optin, pdl_allowed(), dim3(1, p.split), false,
+                                                                           stream, p),
+                       "imma");
 }
 
 template <int kNG>
@@ -397,118 +255,11 @@ int launch_imma_ng(const agb::ImmaParams& p, int wn, int n_tiles, bool bf16, cud
 
 template <int kNG, bool kBf16>
 int launch_imma_persistent_inst(const agb::ImmaPParams& p, int grid, size_t smem, cudaStream_t stream, int smem_optin) {
-  auto kern = agb::w4a16_imma_persistent_kernel<kNG, kBf16>;
-  static bool attr_set_dev[64] = {};   // cudaFuncSetAttribute is per device; benign race: idempotent
-  const int attr_dev = agb::current_device_index();
-  if (!attr_set_dev[attr_dev]) {
-    AGB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_optin));
-    attr_set_dev[attr_dev] = true;
-  }
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(grid, 1, 1);
-  cfg.blockDim = dim3(agb::kIpThreads, 1, 1);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attrs[1];
-  attrs[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attrs[0].val.programmaticStreamSerializationAllowed = pdl_allowed();
-  cfg.attrs = attrs;
-  cfg.numAttrs = 1;
-  AGB_CUDA(cudaLaunchKernelEx(&cfg, kern, p));
-  return 0;
+  return launch_status(agb::launch<agb::w4a16_imma_persistent_kernel<kNG, kBf16>>(dim3(grid), dim3(agb::kIpThreads), smem,
+                                                                                  smem_optin, pdl_allowed(), dim3(1), false,
+                                                                                  stream, p),
+                       "imma persistent");
 }
-
-#ifdef AGB200_EXPERIMENTAL_KERNELS
-template <int kNG, bool kBf16>
-int launch_imma_tma_inst(const agb::ImmaTmaParams& p, const agb::ImmaTmaMaps& maps, int grid, size_t smem, cudaStream_t stream, int smem_optin) {
-  auto kern = agb::w4a16_imma_tma_kernel<kNG, kBf16>;
-  static bool attr_set_dev[64] = {};   // cudaFuncSetAttribute is per device; benign race: idempotent
-  const int attr_dev = agb::current_device_index();
-  if (!attr_set_dev[attr_dev]) {
-    AGB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_optin));
-    attr_set_dev[attr_dev] = true;
-  }
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(grid, 1, 1);
-  cfg.blockDim = dim3(agb::kItThreads, 1, 1);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attrs[1];
-  attrs[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attrs[0].val.programmaticStreamSerializationAllowed = pdl_allowed();
-  cfg.attrs = attrs;
-  cfg.numAttrs = 1;
-  AGB_CUDA(cudaLaunchKernelEx(&cfg, kern, p, maps));
-  return 0;
-}
-
-// TMA-staged persistent form.  Returns 1 when the layer shape is not eligible (caller picks another form).
-int imma_tma_launch(const void* x, int n_layers, const int32_t* const* qweight, const int32_t* const* qzeros, const void* const* scales,
-                    const int32_t* const* perm, const void* const* bias, void* const* y, const int* N, int M, int K, int group_size,
-                    bool bf16, int stages_req, cudaStream_t stream, const DeviceInfo& di) {
-  if (group_size != 128 || K % 128 != 0 || M < 1 || M > agb::kImMaxM) return 1;
-  for (int i = 0; i < n_layers; ++i) {
-    if (N[i] % 32 != 0) return 1;
-    if ((perm ? perm[i] : nullptr) != (perm ? perm[0] : nullptr)) return 1;
-    if (!aligned16(qzeros[i])) return 1;
-  }
-  const int ng = M <= 2 ? 1 : (M <= 5 ? 2 : 3);
-  agb::ImmaTmaParams p{};
-  p.x = x; p.M = M; p.K = K; p.rows = K / 8; p.chunks = (p.rows + agb::kItStageRows - 1) / agb::kItStageRows; p.n_layers = n_layers;
-  const size_t fixed = agb::ImmaTmaSmem::fixed(p.chunks, M, 8 * ng);
-  // as deep as fits: keeping the CTA under half an SM (two layers co-resident under PDL) measured SLOWER than a deeper ring
-  const size_t budget = static_cast<size_t>(di.smem_optin);
-  if (fixed + 2 * agb::kItStageBytes > budget) return 1;
-  int stages = stages_req > 0 ? stages_req : static_cast<int>((budget - fixed) / agb::kItStageBytes);
-  if (stages > agb::kItMaxStages) stages = agb::kItMaxStages;
-  if (stages < 2) stages = 2;
-  if (fixed + static_cast<size_t>(stages) * agb::kItStageBytes > static_cast<size_t>(di.smem_optin)) return 1;
-  p.stages = stages;
-  agb::EncodeTiledFn encode = agb::get_encode_fn();
-  if (encode == nullptr) return fail(AGB200_ECUDA, "cuTensorMapEncodeTiled entry point not available");
-  agb::ImmaTmaMaps maps;
-  memset(&maps, 0, sizeof(maps));
-  const int G = K / 128;
-  int tiles = 0;
-  const cuuint32_t one[2] = {1, 1};
-  for (int i = 0; i < n_layers; ++i) {
-    p.layer[i].qweight = qweight[i]; p.layer[i].qzeros = qzeros[i]; p.layer[i].scales = scales[i];
-    p.layer[i].perm = perm ? perm[i] : nullptr; p.layer[i].bias = bias ? bias[i] : nullptr; p.layer[i].y = y[i];
-    p.layer[i].N = N[i]; p.layer[i].tile_begin = tiles;
-    tiles += N[i] / 32;
-    const cuuint64_t wdim[2] = {static_cast<cuuint64_t>(N[i]), static_cast<cuuint64_t>(p.rows)};
-    const cuuint64_t wstr[1] = {static_cast<cuuint64_t>(N[i]) * 4};
-    const cuuint32_t wbox[2] = {32, static_cast<cuuint32_t>(agb::kItStageRows)};
-    CUresult r1 = encode(&maps.w[i], CU_TENSOR_MAP_DATA_TYPE_INT32, 2, const_cast<int32_t*>(qweight[i]), wdim, wstr, wbox, one,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    const cuuint64_t sdim[2] = {static_cast<cuuint64_t>(N[i]), static_cast<cuuint64_t>(G)};
-    const cuuint64_t sstr[1] = {static_cast<cuuint64_t>(N[i]) * 2};
-    const cuuint32_t sbox[2] = {32, 8};
-    CUresult r2 = encode(&maps.s[i], CU_TENSOR_MAP_DATA_TYPE_UINT16, 2, const_cast<void*>(scales[i]), sdim, sstr, sbox, one,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    const cuuint64_t zdim[2] = {static_cast<cuuint64_t>(N[i] / 8), static_cast<cuuint64_t>(G)};
-    const cuuint64_t zstr[1] = {static_cast<cuuint64_t>(N[i] / 8) * 4};
-    const cuuint32_t zbox[2] = {4, 8};
-    CUresult r3 = encode(&maps.z[i], CU_TENSOR_MAP_DATA_TYPE_INT32, 2, const_cast<int32_t*>(qzeros[i]), zdim, zstr, zbox, one,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r1 != CUDA_SUCCESS || r2 != CUDA_SUCCESS || r3 != CUDA_SUCCESS)
-      return fail(AGB200_ECUDA, "cuTensorMapEncodeTiled failed for layer %d (CUresult %d %d %d)", i, static_cast<int>(r1), static_cast<int>(r2), static_cast<int>(r3));
-  }
-  for (int i = n_layers; i < agb::kGemvMaxGroup; ++i) { maps.w[i] = maps.w[0]; maps.s[i] = maps.s[0]; maps.z[i] = maps.z[0]; }
-  p.total_tiles = tiles;
-  const int grid = tiles < di.sms ? tiles : di.sms;
-  const size_t smem = agb::ImmaTmaSmem::total(stages, p.chunks, M, 8 * ng);
-  switch (ng) {
-    case 1: return bf16 ? launch_imma_tma_inst<1, true>(p, maps, grid, smem, stream, di.smem_optin)
-                        : launch_imma_tma_inst<1, false>(p, maps, grid, smem, stream, di.smem_optin);
-    case 2: return bf16 ? launch_imma_tma_inst<2, true>(p, maps, grid, smem, stream, di.smem_optin)
-                        : launch_imma_tma_inst<2, false>(p, maps, grid, smem, stream, di.smem_optin);
-    default: return bf16 ? launch_imma_tma_inst<3, true>(p, maps, grid, smem, stream, di.smem_optin)
-                         : launch_imma_tma_inst<3, false>(p, maps, grid, smem, stream, di.smem_optin);
-  }
-}
-
-#endif  // AGB200_EXPERIMENTAL_KERNELS
 
 // flush block (k8-rows) of the integer kernel for this layer shape, or 0 when it cannot run it
 int imma_rows_per_block(int K, int group_size) {
@@ -534,19 +285,7 @@ int imma_launch(const void* x, int n_layers, const int32_t* const* qweight, cons
   int tiles32 = 0;
   for (int i = 0; i < n_layers; ++i) tiles32 += (N[i] + 31) / 32;
   const int nblocks = p.rows / rpb;
-  // tune0 (wn_req): 0 = auto, 2 = register-ring persistent form, 3 = TMA-staged persistent form, 1 | 4 = tile-per-CTA form
-  static int form_env = -1;          // measurement aid: AGB200_IMMA_FORM=1|2|3|4 overrides tune0 = 0
-  if (form_env < 0) { const char* e = getenv("AGB200_IMMA_FORM"); form_env = e ? atoi(e) : 0; }
-  if (wn_req == 0 && form_env > 0) wn_req = form_env;
-  if (wn_req == 3) {
-#ifdef AGB200_EXPERIMENTAL_KERNELS
-    const int rc = imma_tma_launch(x, n_layers, qweight, qzeros, scales, perm, bias, y, N, M, K, group_size, bf16, split_req, stream, di);
-    if (rc <= 0) return rc;
-    return fail(AGB200_ENOSUP, "imma TMA form needs group_size == 128, N %% 32 == 0, K %% 128 == 0, one x permutation and room for two stages (K=%d, group_size=%d, M=%d)", K, group_size, M);
-#else
-    return fail(AGB200_ENOSUP, "the TMA-staged IMMA form is an experimental kernel: build with AGB200_EXPERIMENTAL=1");
-#endif
-  }
+  // tune0 (wn_req): 0 = auto, 2 = register-ring persistent form, 1 | 4 = tile-per-CTA form
   // register-ring persistent form (one 512-thread CTA per SM): 128-k flush blocks and one x permutation for all sibling
   // layers; x is converted per K chunk when its digits do not fit in shared memory at once
   {
@@ -559,13 +298,7 @@ int imma_launch(const void* x, int n_layers, const int32_t* const* qweight, cons
       agb::ImmaPParams q{};
       q.x = x; q.M = M; q.K = K; q.rows = p.rows; q.blocks_per_group = p.rows_per_group / rpb; q.n_layers = n_layers;
       q.pf = take_prefetch_hint();
-      int tiles = 0;
-      for (int i = 0; i < n_layers; ++i) {
-        q.layer[i].qweight = qweight[i]; q.layer[i].qzeros = qzeros[i]; q.layer[i].scales = scales[i];
-        q.layer[i].perm = perm ? perm[i] : nullptr; q.layer[i].bias = bias ? bias[i] : nullptr; q.layer[i].y = y[i];
-        q.layer[i].N = N[i]; q.layer[i].tile_begin = tiles;
-        tiles += (N[i] + 31) / 32;
-      }
+      const int tiles = fill_layers(q.layer, n_layers, qweight, qzeros, scales, perm, bias, y, N, 32);
       q.total_tiles = tiles;
       const int grid = tiles < di.sms ? tiles : di.sms;
       agb::prefetch_set_grid(q.pf, static_cast<unsigned>(grid));
@@ -610,13 +343,7 @@ int imma_launch(const void* x, int n_layers, const int32_t* const* qweight, cons
   if (wn != 1 && wn != 4) return fail(AGB200_EINVAL, "imma: tune0 must be 0 (auto), 1 or 4 (warps along N of the tile-per-CTA kernel) or 2 (persistent); got %d", wn);
   p.split = split;
   p.rows_per_split = rps_of(split);
-  int tiles = 0;
-  for (int i = 0; i < n_layers; ++i) {
-    p.layer[i].qweight = qweight[i]; p.layer[i].qzeros = qzeros[i]; p.layer[i].scales = scales[i];
-    p.layer[i].perm = perm ? perm[i] : nullptr; p.layer[i].bias = bias ? bias[i] : nullptr; p.layer[i].y = y[i];
-    p.layer[i].N = N[i]; p.layer[i].tile_begin = tiles;
-    tiles += (N[i] + 32 * wn - 1) / (32 * wn);
-  }
+  const int tiles = fill_layers(p.layer, n_layers, qweight, qzeros, scales, perm, bias, y, N, 32 * wn);
   switch (ng) {
     case 1: return launch_imma_ng<1>(p, wn, tiles, bf16, stream, di.smem_optin);
     case 2: return launch_imma_ng<2>(p, wn, tiles, bf16, stream, di.smem_optin);
@@ -638,6 +365,18 @@ int check_common(const void* x, const int32_t* qweight, const int32_t* qzeros, c
   return 0;
 }
 
+// Runs pass(x rows, y rows, m) over the M rows of x [M, K] and y [M, N] in passes of at most `rows` rows; stops at the
+// first pass that fails.
+template <typename Pass>
+int in_row_passes(const void* x, void* y, int M, int K, int N, int rows, Pass&& pass) {
+  const size_t xs = static_cast<size_t>(K) * 2, ys = static_cast<size_t>(N) * 2;
+  for (int m0 = 0; m0 < M; m0 += rows) {
+    const int m = (M - m0 < rows) ? (M - m0) : rows;
+    if (int rc = pass(static_cast<const char*>(x) + m0 * xs, static_cast<char*>(y) + m0 * ys, m)) return rc;
+  }
+  return 0;
+}
+
 }  // namespace
 
 int agb_internal_fail(int code, const char* msg) { return fail(code, "%s", msg); }
@@ -651,11 +390,7 @@ const char* agb200_build_info(void) {
   return "autogptq_b200 sm_100a: decode=IMMA.16832.U8.S8 on raw nibbles x block-fixed-point activations (M<=8) + PDL; "
          "gemv=cuda-core FHFMA (fma.rn.f32.f16) + cluster/DSMEM split-K; "
          "gemm=tcgen05.mma kind::f16 (A=dequantised W^T in TMEM, B=x via TMA SWIZZLE_128B), fp32 TMEM accumulators; "
-         "chain=persistent TMA ring + IMMA consumers + tagged-word dependencies"
-#ifdef AGB200_EXPERIMENTAL_KERNELS
-         "; experimental=decode_tma,decode_tc,decode_imma_tma"
-#endif
-      ;
+         "chain=persistent TMA ring + IMMA consumers + tagged-word dependencies";
 }
 
 int agb200_w4_prefetch_hint(int n, const void* const* ptrs, const size_t* bytes) {
@@ -711,89 +446,21 @@ int agb200_w4a16_forward_ex(const void* x, const int32_t* qweight, const int32_t
     else if (!gemm_ok || (M <= AGB200_SKINNY_MAX_M && !huge)) kernel = AGB200_KERNEL_SKINNY;     // passes of 8 rows
     // (5..8 rows on >= 100 MB layers: the 32-row tcgen05 tile is ahead of the skinny kernel, 65-69 us vs 83-100 us)
     else kernel = AGB200_KERNEL_GEMM;
-    if (M <= AGB200_SKINNY_MAX_M && tc_ok) {
-      static int forced = -1;                                             // measurement aid: AGB200_SMALL_M_KERNEL=1|3|4|6
-      if (forced < 0) { const char* e = getenv("AGB200_SMALL_M_KERNEL"); forced = e ? atoi(e) : 0; }
-      #ifdef AGB200_EXPERIMENTAL_KERNELS
-      if (forced == AGB200_KERNEL_DECODE) kernel = forced;
-#endif
-      if (forced == AGB200_KERNEL_GEMV || forced == AGB200_KERNEL_SKINNY) kernel = forced;
-      if (forced == AGB200_KERNEL_IMMA && imma_ok) kernel = forced;
-    }
   }
-  if (kernel == AGB200_KERNEL_IMMA) {
-    const size_t xs = static_cast<size_t>(K) * 2, ys = static_cast<size_t>(N) * 2;
-    for (int m0 = 0; m0 < M; m0 += agb::kImMaxM) {
-      const int m = (M - m0 < agb::kImMaxM) ? (M - m0) : agb::kImMaxM;
-      void* ypp = static_cast<char*>(y) + m0 * ys;
-      if (int rc = imma_launch(static_cast<const char*>(x) + m0 * xs, 1, &qweight, &qzeros, &scales, &perm, &bias, &ypp, &N,
-                               m, K, group_size, bf16, tune0, tune1, stream, di))
-        return rc;
-    }
-    return 0;
-  }
-#ifndef AGB200_EXPERIMENTAL_KERNELS
-  if (kernel == AGB200_KERNEL_DECODE || kernel == AGB200_KERNEL_TCDECODE)
-    return fail(AGB200_ENOSUP, "kernel %d is an experimental kernel that AUTO never selects: build with AGB200_EXPERIMENTAL=1", kernel);
-#else
-  if (kernel == AGB200_KERNEL_DECODE) {
-    const size_t xs = static_cast<size_t>(K) * 2, ys = static_cast<size_t>(N) * 2;
-    // shared memory holds all of x: fall back to the cluster split-K kernel when K x M does not fit
-    const bool fits = agb::DecodeSmem::total(2, K / 8, M < 8 ? M : 8) <= static_cast<size_t>(di.smem_optin);
-    if (fits) {
-      for (int m0 = 0; m0 < M; m0 += agb::kDcMaxM) {
-        const int m = (M - m0 < agb::kDcMaxM) ? (M - m0) : agb::kDcMaxM;
-        if (int rc = decode_launch(static_cast<const char*>(x) + m0 * xs, qweight, qzeros, scales, perm, bias,
-                                   static_cast<char*>(y) + m0 * ys, m, K, N, group_size, bf16, tune0, tune1, stream, di))
-          return rc;
-      }
-      return 0;
-    }
-    kernel = AGB200_KERNEL_SKINNY;
-  }
-#endif
-  if (kernel == AGB200_KERNEL_SKINNY) {
-    const bool biased = (flags & 1) != 0 && !bf16;
-    const size_t xs = static_cast<size_t>(K) * 2, ys = static_cast<size_t>(N) * 2;
-    for (int m0 = 0; m0 < M; m0 += AGB200_SKINNY_MAX_M) {
-      const int m = (M - m0 < AGB200_SKINNY_MAX_M) ? (M - m0) : AGB200_SKINNY_MAX_M;
-      if (int rc = skinny_launch(static_cast<const char*>(x) + m0 * xs, qweight, qzeros, scales, perm, bias,
-                                 static_cast<char*>(y) + m0 * ys, m, K, N, group_size, bf16, tune1, biased, stream, di))
-        return rc;
-    }
-    return 0;
-  }
-
-  if (kernel == AGB200_KERNEL_GEMV) {
-    const bool biased = (flags & 1) != 0 && !bf16;
-    const size_t xs = static_cast<size_t>(K) * 2, ys = static_cast<size_t>(N) * 2;
-    for (int m0 = 0; m0 < M; m0 += AGB200_GEMV_MAX_M) {
-      const int m = (M - m0 < AGB200_GEMV_MAX_M) ? (M - m0) : AGB200_GEMV_MAX_M;
-      if (int rc = gemv_pass(static_cast<const char*>(x) + m0 * xs, qweight, qzeros, scales, perm, bias,
-                             static_cast<char*>(y) + m0 * ys, m, K, N, group_size, bf16, tune0, tune1, biased, stream, di, (flags >> 4) & 7))
-        return rc;
-    }
-    return 0;
-  }
-#ifdef AGB200_EXPERIMENTAL_KERNELS
-  if (kernel == AGB200_KERNEL_TCDECODE) {
-    if (qweight_tc == nullptr)
-      return fail(AGB200_ENOSUP, "the tcgen05 decode kernel needs qweight_tc: run agb200_w4_prepare_tc once at load time");
-    const size_t xs = static_cast<size_t>(K) * 2, ys = static_cast<size_t>(N) * 2;
-    for (int m0 = 0; m0 < M; m0 += agb::kTdMT) {
-      agb::GemmArgs a{};
-      a.x = static_cast<const char*>(x) + m0 * xs; a.qweight = qweight_tc; a.qzeros = qzeros; a.scales = scales; a.perm = perm;
-      a.bias = bias; a.y = static_cast<char*>(y) + m0 * ys;
-      a.M = (M - m0 < agb::kTdMT) ? (M - m0) : agb::kTdMT; a.K = K; a.N = N; a.group_size = group_size; a.bf16 = bf16;
-      a.workspace = workspace; a.workspace_bytes = workspace_bytes;
-      a.split_k = tune1; a.sms = di.sms; a.smem_optin = di.smem_optin;
-      char msg[400] = "";
-      const int rc = agb::launch_w4a16_tcdecode(a, pdl_allowed(), stream, msg, sizeof(msg));
-      if (rc != 0) return fail(rc, "%s", msg);
-    }
-    return 0;
-  }
-#endif
+  const bool biased = (flags & 1) != 0 && !bf16;
+  if (kernel == AGB200_KERNEL_IMMA)
+    return in_row_passes(x, y, M, K, N, agb::kImMaxM, [&](const void* xp, void* yp, int m) {
+      return imma_launch(xp, 1, &qweight, &qzeros, &scales, &perm, &bias, &yp, &N, m, K, group_size, bf16, tune0, tune1, stream, di);
+    });
+  if (kernel == AGB200_KERNEL_SKINNY)
+    return in_row_passes(x, y, M, K, N, AGB200_SKINNY_MAX_M, [&](const void* xp, void* yp, int m) {
+      return skinny_launch(xp, qweight, qzeros, scales, perm, bias, yp, m, K, N, group_size, bf16, tune1, biased, stream, di);
+    });
+  if (kernel == AGB200_KERNEL_GEMV)
+    return in_row_passes(x, y, M, K, N, AGB200_GEMV_MAX_M, [&](const void* xp, void* yp, int m) {
+      return gemv_pass(xp, qweight, qzeros, scales, perm, bias, yp, m, K, N, group_size, bf16, tune0, tune1, biased, stream, di,
+                       (flags >> 4) & 7);
+    });
   if (kernel == AGB200_KERNEL_GEMM) {
     if (qweight_tc == nullptr)
       return fail(AGB200_ENOSUP, "the tensor-core path (M=%d > 8) needs qweight_tc: run agb200_w4_prepare_tc once at load time", M);
@@ -825,12 +492,9 @@ int agb200_w4a16_forward_group(const void* x, int n_layers, const int32_t* const
   DeviceInfo di;
   if (int rc = get_device_info(di)) return rc;
   {
-    static int forced = -1;
-    if (forced < 0) { const char* e = getenv("AGB200_SMALL_M_KERNEL"); forced = e ? atoi(e) : 0; }
     bool same_perm = true;
     for (int i = 1; i < n_layers; ++i) same_perm = same_perm && (perm ? perm[i] : nullptr) == (perm ? perm[0] : nullptr);
-    const bool imma_ok = imma_rows_per_block(K, group_size) == 16 && same_perm && n_layers > 1 && M <= agb::kImMaxM;
-    if (imma_ok && ((forced == 0 && M >= 2 && M <= 4) || forced == AGB200_KERNEL_IMMA))
+    if (M >= 2 && M <= 4 && n_layers > 1 && same_perm && imma_rows_per_block(K, group_size) == 16)
       return imma_launch(x, n_layers, qweight, qzeros, scales, perm, bias, y, N, M, K, group_size, dtype == AGB200_BF16, 0, 0,
                          static_cast<cudaStream_t>(stream_), di);
   }
@@ -847,13 +511,7 @@ int agb200_w4a16_forward_group(const void* x, int n_layers, const int32_t* const
   p.n_group = n_layers;
   p.pf = take_prefetch_hint();
   constexpr int kLN = 8;
-  int tiles = 0;
-  for (int i = 0; i < n_layers; ++i) {
-    p.group[i].qweight = qweight[i]; p.group[i].qzeros = qzeros[i]; p.group[i].scales = scales[i];
-    p.group[i].perm = perm ? perm[i] : nullptr; p.group[i].bias = bias ? bias[i] : nullptr; p.group[i].y = y[i];
-    p.group[i].N = N[i]; p.group[i].tile_begin = tiles;
-    tiles += (N[i] + kLN * 4 - 1) / (kLN * 4);
-  }
+  const int tiles = fill_layers(p.group, n_layers, qweight, qzeros, scales, perm, bias, y, N, kLN * 4);
   p.N = N[0];
   // same tiling rules as the single-layer GEMV, applied to the whole group (32-column CTAs)
   int split = (tiles >= 192 || p.rows <= 768) ? 1 : 2;

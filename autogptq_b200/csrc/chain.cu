@@ -106,25 +106,12 @@ const char* site_name(int site) {
 
 template <int kM, bool kBf16, bool kProf>
 int launch_inst(const Chain& c, int flags, cudaStream_t stream) {
-  auto kern = agb::w4a16_chain_kernel<kM, kBf16, kProf>;
-  static bool attr_set[64] = {};
-  if (!attr_set[c.device]) {
-    CH_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, c.smem_optin));
-    attr_set[c.device] = true;
-  }
   agb::ChainParams p = c.params;
   p.debug = flags;
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(c.grid, 1, 1);
-  cfg.blockDim = dim3(agb::kChThreads, 1, 1);
-  cfg.dynamicSmemBytes = c.smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attrs[1];
-  attrs[0].id = cudaLaunchAttributeCooperative;      // every CTA must be resident: they wait for each other's outputs
-  attrs[0].val.cooperative = 1;
-  cfg.attrs = attrs;
-  cfg.numAttrs = 1;
-  CH_CUDA(cudaLaunchKernelEx(&cfg, kern, p));
+  // cooperative: every CTA must be resident, they wait for each other's outputs
+  const cudaError_t e = agb::launch<agb::w4a16_chain_kernel<kM, kBf16, kProf>>(dim3(c.grid), dim3(agb::kChThreads), c.smem,
+                                                                              c.smem_optin, false, dim3(1), true, stream, p);
+  if (e != cudaSuccess) return failf(AGB200_ECUDA, "chain launch: %s", cudaGetErrorString(e));
   return 0;
 }
 

@@ -5,16 +5,58 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <atomic>
+
 namespace agb {
 
 constexpr int kPack = 8;  // nibbles per int32 word of qweight / qzeros
 
-// Index into the per-device "function attribute already set" tables of the launchers (the opt-in to > 48 KB of dynamic
-// shared memory is per device: a process that drives several GPUs must set it on each of them).
-inline int current_device_index() {
-  int d = 0;
-  if (cudaGetDevice(&d) != cudaSuccess || d < 0 || d >= 64) d = 0;
-  return d;
+// ---------------------------------------------------------------- host: kernel launch
+// Every kernel of the library is launched here.  `smem_optin` is the dynamic shared memory the kernel is allowed to
+// use; the opt-in is per device (a process that drives several GPUs must make it on each of them), so it is made on the
+// first launch of `kKernel` on each device (on every launch beyond device 63).  The flags are keyed on the kernel
+// itself, not on its signature: template instances with the same parameter types each have their own.  The cluster
+// attribute is set when `cluster` holds more than one CTA.
+template <auto kKernel, typename... Args>
+cudaError_t launch(dim3 grid, dim3 block, size_t smem, int smem_optin, bool pdl, dim3 cluster, bool cooperative,
+                   cudaStream_t stream, const Args&... args) {
+  static std::atomic<bool> optin_done[64];
+  int dev = 0;
+  cudaError_t e = cudaGetDevice(&dev);
+  if (e != cudaSuccess) return e;
+  const bool cached = dev >= 0 && dev < 64;
+  if (!cached || !optin_done[dev].load(std::memory_order_acquire)) {
+    e = cudaFuncSetAttribute(kKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_optin);
+    if (e != cudaSuccess) return e;
+    if (cached) optin_done[dev].store(true, std::memory_order_release);
+  }
+  cudaLaunchAttribute attrs[3];
+  int na = 0;
+  if (pdl) {
+    attrs[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attrs[na].val.programmaticStreamSerializationAllowed = 1;
+    ++na;
+  }
+  if (cluster.x * cluster.y * cluster.z > 1) {
+    attrs[na].id = cudaLaunchAttributeClusterDimension;
+    attrs[na].val.clusterDim.x = cluster.x;
+    attrs[na].val.clusterDim.y = cluster.y;
+    attrs[na].val.clusterDim.z = cluster.z;
+    ++na;
+  }
+  if (cooperative) {   // every CTA is resident at once
+    attrs[na].id = cudaLaunchAttributeCooperative;
+    attrs[na].val.cooperative = 1;
+    ++na;
+  }
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = grid;
+  cfg.blockDim = block;
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = stream;
+  cfg.attrs = attrs;
+  cfg.numAttrs = na;
+  return cudaLaunchKernelEx(&cfg, kKernel, args...);
 }
 
 // ---------------------------------------------------------------- memory

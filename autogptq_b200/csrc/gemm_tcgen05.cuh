@@ -411,36 +411,16 @@ inline size_t gemm_workspace_bytes(int M, int K, int) {
 template <int kMT, bool kBf16, bool kMcast>
 int launch_gemm_inst(const GemmParams& p, const CUtensorMap& tmap, const CUtensorMap& tmap_w, const CUtensorMap& tmap_s,
                      const CUtensorMap& tmap_z, int m_tiles, cudaStream_t stream, char* msg, size_t msg_n) {
-  auto kern = w4a16_gemm_kernel<kMT, kBf16, kMcast>;
   constexpr int smem = GemmSmem<kMT>::kTotal;
-  static bool attr_set_dev[64] = {};   // cudaFuncSetAttribute is per device; benign race: idempotent
-  const int attr_dev = agb::current_device_index();
-  if (!attr_set_dev[attr_dev]) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    if (e != cudaSuccess) { snprintf(msg, msg_n, "gemm: cudaFuncSetAttribute(%d B): %s", smem, cudaGetErrorString(e)); return -2; }
-    attr_set_dev[attr_dev] = true;
+  // cluster: a 2x1 pair that shares the multicast x tile, or the split-K CTAs of one output tile along z
+  const dim3 cluster = kMcast ? dim3(2, 1, 1) : dim3(1, 1, p.split);
+  cudaError_t e = launch<w4a16_gemm_kernel<kMT, kBf16, kMcast>>(dim3((p.N + kGemmBN - 1) / kGemmBN, m_tiles, p.split),
+                                                               dim3(gemm_threads(kMT)), smem, smem, true, cluster, false,
+                                                               stream, p, tmap, tmap_w, tmap_s, tmap_z);
+  if (e != cudaSuccess) {
+    snprintf(msg, msg_n, "gemm launch (MT=%d split=%d, %d B shared memory): %s", kMT, p.split, smem, cudaGetErrorString(e));
+    return -2;
   }
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((p.N + kGemmBN - 1) / kGemmBN, m_tiles, p.split);
-  cfg.blockDim = dim3(gemm_threads(kMT), 1, 1);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attrs[2];
-  int na = 0;
-  attrs[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attrs[na].val.programmaticStreamSerializationAllowed = 1;
-  ++na;
-  if (p.split > 1 || kMcast) {
-    attrs[na].id = cudaLaunchAttributeClusterDimension;
-    attrs[na].val.clusterDim.x = kMcast ? 2 : 1;
-    attrs[na].val.clusterDim.y = 1;
-    attrs[na].val.clusterDim.z = kMcast ? 1 : p.split;
-    ++na;
-  }
-  cfg.attrs = attrs;
-  cfg.numAttrs = na;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, p, tmap, tmap_w, tmap_s, tmap_z);
-  if (e != cudaSuccess) { snprintf(msg, msg_n, "gemm launch (MT=%d split=%d): %s", kMT, p.split, cudaGetErrorString(e)); return -2; }
   return 0;
 }
 

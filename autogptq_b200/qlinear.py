@@ -221,7 +221,7 @@ class QuantLinear(nn.Module):
         ws_ptr, ws_bytes, p_tc = None, 0, None
         if M > 4 or self.kernel != _lib.KERNEL_AUTO:
             big_m = M > _lib.IMMA_MAX_M or (M >= 5 and K * N >= 1.0e8 and not (M == 5 and self.group_size % 128 == 0 and K % 128 == 0))
-            needs_tc = self.kernel in (_lib.KERNEL_GEMM, _lib.KERNEL_TCDECODE) or (
+            needs_tc = self.kernel == _lib.KERNEL_GEMM or (
                 self.kernel == _lib.KERNEL_AUTO and big_m and (self.group_size == 32 or self.group_size % 64 == 0) and N % 32 == 0)
             if needs_tc:
                 if self._qweight_tc is None:

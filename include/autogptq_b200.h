@@ -54,8 +54,7 @@ extern "C" {
 #define AGB200_KERNEL_GEMV 1   /* CUDA-core FHFMA GEMV, M <= AGB200_GEMV_MAX_M per pass (AUTO: M = 1) */
 #define AGB200_KERNEL_GEMM 2   /* tcgen05 / TMEM tensor-core GEMM */
 #define AGB200_KERNEL_SKINNY 3 /* decode batches M <= 8: warp-level MMA on subnormal-encoded nibbles, cluster split-K (AUTO: M = 5..8) */
-#define AGB200_KERNEL_DECODE 4 /* experimental: M <= 8, TMA-staged persistent CTAs (not picked by AUTO; AGB200_ENOSUP unless the library was built with -DAGB200_EXPERIMENTAL_KERNELS) */
-#define AGB200_KERNEL_TCDECODE 5 /* experimental: M <= 16 on tcgen05, unpack-only + per-group TMEM accumulators (needs qweight_tc; not picked by AUTO; same build flag) */
+/* 4 and 5 are unused (they named kernels that were removed); a caller that passes them gets AGB200_EINVAL */
 #define AGB200_KERNEL_IMMA 6 /* decode batches M <= 8: integer tensor cores on raw nibbles, x as 24-bit block fixed point (AUTO: M = 2..4) */
 #define AGB200_GEMV_MAX_M 4
 #define AGB200_SKINNY_MAX_M 8
@@ -106,9 +105,7 @@ int agb200_w4a16_forward(const void* x, const int32_t* qweight, const int32_t* q
  *   tune0/1  GEMV: tune0 = lanes along N per warp (8|16|32, 0=auto), tune1 = split-K (1|2|4|8, 0=auto),
  *            flags bit0 = biased-exponent unpack instead of the subnormal unpack.
  *            SKINNY: tune1 = split-K (1|2|4|8, 0=auto), flags bit0 as for GEMV.
- *            DECODE: tune0 = grid size (0=auto), tune1 = ring stages (2..8, 0=auto).
- *            TCDECODE: tune1 = split-K (1|2|4|8, 0=auto).
- *            IMMA: tune0 = 0 auto | 3 TMA-staged persistent form | 2 register-ring persistent form | 1, 4 tile-per-CTA form
+ *            IMMA: tune0 = 0 auto | 2 register-ring persistent form | 1, 4 tile-per-CTA form
  *                  with that many warps along N;
  *                  tune1 = split-K of the tile-per-CTA form (1|2|4|8, 0=auto).
  *            GEMM: tune0 = x-row tile (16..256, 0=auto), tune1 = split-K (0=auto). */

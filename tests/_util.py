@@ -65,12 +65,3 @@ def digest(*arrays) -> str:
 def rand_x(M, K, seed=1, dtype=np.float16):
     return np.random.default_rng(seed).standard_normal((M, K)).astype(np.float32).astype(dtype)
 
-
-def experimental_kernels_built() -> bool:
-    """True when the library contains the three decode kernel families AUTO never selects (AGB200_EXPERIMENTAL=1 build)."""
-    try:
-        from autogptq_b200 import _lib
-
-        return b"experimental=" in _lib.load().agb200_build_info()
-    except Exception:
-        return False

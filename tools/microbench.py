@@ -95,7 +95,7 @@ def main():
     ap.add_argument("--sweep5", action="store_true",
                     help="BASELINE.json configs[4]: M in {1,8,64,512} x (K,N) in {4096,11008}^2 x g in {32,128,-1}, AUTO vs the reference kernels")
     ap.add_argument("--out", default="gpurun_out/micro.jsonl")
-    ap.add_argument("--what", default="auto,imma,gemv,skinny,decode,tcd,gemm,ref")
+    ap.add_argument("--what", default="auto,imma,gemv,skinny,gemm,ref")
     args = ap.parse_args()
     global HBM_PEAK, TF_PEAK
     try:
@@ -145,7 +145,7 @@ def main():
             for M in (1, 2, 3, 4, 5, 8):
                 variants = [(0, 0, 0)]
                 if M in (1, 2, 4):
-                    variants += [(3, 0, 0), (2, 0, 0)]
+                    variants += [(2, 0, 0)]
                 for tune in variants:
                     try:
                         med, mn = time_config(lib, L, M, 6, tune)
@@ -182,32 +182,6 @@ def main():
                         continue
                     ab = alg_bytes(M, K, N, g)
                     emit({"kernel": "skinny", "K": K, "N": N, "g": g, "M": M, "tune": tune, "us": round(med, 3), "us_min": round(mn, 3),
-                          "GBps": round(ab / med / 1e3, 1), "hbm_frac": round(ab / med / 1e3 / HBM_PEAK, 3)})
-        if "decode" in args.what:
-            for M in (1, 2, 4, 8):
-                variants = [(0, 0, 0)]
-                if M == 1:
-                    variants += [(gr, st, 0) for gr in (0, 64, 128, 148) for st in (2, 3, 4, 6)]
-                for tune in variants:
-                    try:
-                        med, mn = time_config(lib, L, M, 4, tune)
-                    except Exception as e:
-                        emit({"kernel": "decode", "K": K, "N": N, "g": g, "M": M, "tune": tune, "error": str(e)})
-                        continue
-                    ab = alg_bytes(M, K, N, g)
-                    emit({"kernel": "decode", "K": K, "N": N, "g": g, "M": M, "tune": tune, "us": round(med, 3), "us_min": round(mn, 3),
-                          "GBps": round(ab / med / 1e3, 1), "hbm_frac": round(ab / med / 1e3 / HBM_PEAK, 3)})
-        if "tcd" in args.what:
-            for M in (1, 4, 8, 16):
-                variants = [(0, 0, 0)] + ([(0, sp, 0) for sp in (1, 2, 4, 8)] if M == 1 else [])
-                for tune in variants:
-                    try:
-                        med, mn = time_config(lib, L, M, 5, tune)
-                    except Exception as e:
-                        emit({"kernel": "tcdecode", "K": K, "N": N, "g": g, "M": M, "tune": tune, "error": str(e)})
-                        continue
-                    ab = alg_bytes(M, K, N, g)
-                    emit({"kernel": "tcdecode", "K": K, "N": N, "g": g, "M": M, "tune": tune, "us": round(med, 3), "us_min": round(mn, 3),
                           "GBps": round(ab / med / 1e3, 1), "hbm_frac": round(ab / med / 1e3 / HBM_PEAK, 3)})
         if "gemm" in args.what:
             for M in ((16, 64, 128, 512, 2048, 16384) if not args.quick else (16, 64, 512, 4096)):

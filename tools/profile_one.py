@@ -1,4 +1,4 @@
-"""Launch one configuration a few times (for ncu).  usage: profile_one.py {gemv|gemm|skinny|decode|tcd|imma} K N M [tune0 tune1 tune2]"""
+"""Launch one configuration a few times (for ncu).  usage: profile_one.py {gemv|gemm|skinny|imma} K N M [tune0 tune1 tune2]"""
 import sys, os
 import torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -14,7 +14,7 @@ y = torch.empty(M, N, dtype=torch.float16, device="cuda")
 for it in range(2):
     for c in range(L.copies):
         rc = lib.agb200_w4a16_forward_ex(x.data_ptr(), L.qw[c].data_ptr(), L.qw_tc[c].data_ptr(), L.qz[c].data_ptr(), L.sc[c].data_ptr(), None, None,
-                                         y.data_ptr(), M, K, N, 128, 0, None, 0, None, {"gemv": 1, "gemm": 2, "skinny": 3, "decode": 4, "tcd": 5, "imma": 6}[kind], *tune)
+                                         y.data_ptr(), M, K, N, 128, 0, None, 0, None, {"gemv": 1, "gemm": 2, "skinny": 3, "imma": 6}[kind], *tune)
         assert rc == 0, lib.agb200_last_error()
 torch.cuda.synchronize()
 print("ok")
