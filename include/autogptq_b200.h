@@ -243,8 +243,9 @@ int agb200_w4_prefetch_hint(int n, const void* const* ptrs, const size_t* bytes)
 /*
  * End-to-end variant with HOST activations: copies x_host -> device staging, runs the forward
  * and copies y back to y_host, all on `stream` (asynchronous when the host buffers are pinned).
- * `staging` is device scratch of agb200_w4a16_host_staging_bytes(M,K,N) bytes.
- * This is the call `bench.py` times for the "e2e" number.
+ * `staging` is device scratch of agb200_w4a16_host_staging_bytes(M,K,N) bytes: x, y and the forward's workspace are
+ * carved from it, so act-order layers on the tensor-core path need no other buffer.  A smaller buffer returns
+ * AGB200_EWORKSPACE before anything is copied or launched.  Pageable host buffers make the copies synchronous.
  */
 int agb200_w4a16_forward_host(const void* x_host, const int32_t* qweight, const int32_t* qweight_tc, const int32_t* qzeros,
                               const void* scales, const int32_t* perm, const void* bias, void* y_host,

@@ -38,6 +38,44 @@ def oracle_fp16w(d, x):
     return y
 
 
+def _round16(a, dtype):
+    """float32 values of `a` rounded (nearest-even) to the 16-bit torch dtype."""
+    return torch.from_numpy(np.ascontiguousarray(a, dtype=np.float32)).to(dtype).float().numpy()
+
+
+def round_layer(d, dtype):
+    """Round `scales` and `bias` of an oracle layer to the 16-bit type `dtype`, in place, so that the kernel (which
+    stores them in that type) and the oracle see the same numbers.  Returns d."""
+    d["scales"] = _round16(d["scales"], dtype)
+    if d.get("bias") is not None:
+        d["bias"] = _round16(d["bias"], dtype)
+    return d
+
+
+def slice_cols(d, n0, n1):
+    """The oracle layer restricted to output columns [n0, n1) (multiples of 8): every column is independent, so a
+    slice keeps the host oracle of a full-size layer cheap."""
+    out = dict(d)
+    out.update(qweight=d["qweight"][:, n0:n1], qzeros=d["qzeros"][:, n0 // 8:n1 // 8], scales=d["scales"][:, n0:n1], N=n1 - n0)
+    if d.get("bias") is not None:
+        out["bias"] = np.asarray(d["bias"])[n0:n1]
+    return out
+
+
+def oracle_wround(d, x, dtype=torch.float16):
+    """Tensor-core path arithmetic: W = rn_dtype(s * (q - z)) rounded once to the 16-bit type, fp32 accumulate.
+    (s * (q - z) is exact in fp32 for 16-bit s and |q - z| <= 15, so the only rounding is the one to `dtype`.)"""
+    q = O.unpack_qweight(d["qweight"]).astype(np.float32)
+    z = O.unpack_qzeros(d["qzeros"]).astype(np.float32)
+    g = np.asarray(d["g_idx"]).astype(np.int64)
+    s = np.asarray(d["scales"], dtype=np.float32)
+    W = _round16(s[g] * (q - z[g]), dtype)
+    y = np.asarray(x, dtype=np.float32).reshape(-1, W.shape[0]) @ W
+    if d.get("bias") is not None:
+        y = y + np.asarray(d["bias"], dtype=np.float32)
+    return y
+
+
 def assert_parity(y, y_ref, rtol=1e-3, atol_rms=1e-3, what=""):
     """north_star tolerance: 1e-3 relative in fp16.  |y - ref| <= rtol*|ref| + atol_rms*rms(ref) elementwise,
     and max|y - ref| <= 1e-3 * max|ref| (SURVEY Appendix A)."""

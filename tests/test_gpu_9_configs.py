@@ -15,23 +15,15 @@ import pytest
 import torch
 
 from oracle import w4a16_oracle as O
-from tests._util import assert_parity, make_layer, rand_x
+from tests._util import assert_parity, make_layer, oracle_exact, oracle_fp16w, rand_x, slice_cols
 
 pytestmark = pytest.mark.gpu
 
 
 def _oracle_cols(d, x, n0, n1, fp16_w=False):
-    """Exact oracle on output columns [n0, n1) (multiples of 8)."""
-    qw, qz, sc = d["qweight"][:, n0:n1], d["qzeros"][:, n0 // 8:n1 // 8], d["scales"][:, n0:n1]
-    if fp16_w:
-        W = O.dequantize(qw, qz, sc, g_idx=d["g_idx"], group_size=d["group_size"], dtype=np.float16).astype(np.float32)
-        y = np.asarray(x, dtype=np.float32) @ W
-    else:
-        y = O.forward(np.asarray(x, dtype=np.float32), qw, qz, sc, g_idx=d["g_idx"], group_size=d["group_size"], bias=None,
-                      out_dtype=np.float32)
-    if d.get("bias") is not None:
-        y = y + np.asarray(d["bias"], dtype=np.float32)[n0:n1]
-    return y
+    """Exact (or fp16-W) oracle on output columns [n0, n1) (multiples of 8)."""
+    ds = slice_cols(d, n0, n1)
+    return oracle_fp16w(ds, x) if fp16_w else oracle_exact(ds, x)
 
 
 def _slice_for(N, seed, width=256):
